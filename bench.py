@@ -1,6 +1,7 @@
 """bench.py — decode tokens/sec of the soft-attention LSTM decode path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl sat|reference] [--workload 2|3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl sat|reference] [--workload 2|3|4|5]
+                    [--dump-outputs DIR]
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 A "step" is one pass of the hot path over one batch of synthetic contexts: project the
@@ -150,6 +151,18 @@ def loop_kernel_times(model, ctx, T, work, pk):
     return out
 
 
+def dump_outputs(directory, arrays):
+    """Write what the timed path returned in its last step as <directory>/<name>.npy: float64 stays float64, every
+    other type becomes float32 (token ids < 2**24 are exact).  Inputs and weights are seeded, so two builds run with
+    the same arguments can be compared output for output: two runs of one build give bit-identical greedy and beam
+    outputs, and training losses that agree to fp32 round-off.  Every workload's outputs are far below 64 MB."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
+
+
 def oracle_setup(wl, seed=1234):
     from oracle import ref_step as R
     ocfg = R.OracleConfig(batch_size=wl["B"], num_ctx=wl["L"], dim_ctx=wl["D"], num_lstm_units=wl["H"],
@@ -246,9 +259,10 @@ def run_reference(args, wl, rank, world):
     print(json.dumps(line), flush=True)
 
 
-def measure_training(wl, model, rank, local_rank, world, dev, steps, warmup, e2e=True, sample_clocks=True):
+def measure_training(wl, model, rank, local_rank, world, dev, steps, warmup, e2e=True, sample_clocks=True, dump=None):
     """config 4: one optimisation step per bench step (forward + backward + gradient all-reduce + clip + Adam); weak
-    scaling, 64 images per GPU.  Returns the record (rank 0) or None."""
+    scaling, 64 images per GPU.  dump: directory for the losses and squared gradient norm of the last timed step.
+    Returns the record (rank 0) or None."""
     import torch
     import torch.distributed as dist
     from sat_b200 import parallel
@@ -280,9 +294,11 @@ def measure_training(wl, model, rank, local_rank, world, dev, steps, warmup, e2e
     with torch.cuda.stream(st):
         ev0.record(st)
         for i in range(steps):
-            model.train_step(ctx_dev[i % pool], sent, masks, seed=100 + i, sync=False)   # losses stay on the device
+            last = model.train_step(ctx_dev[i % pool], sent, masks, seed=100 + i, sync=False)   # losses stay on the device
         ev1.record(st)
     barrier()
+    if dump and rank == 0:
+        dump_outputs(dump, dict(losses=last[0], gradient_norm_squared=last[1]))
     ms = parallel.max_over_ranks(ev0.elapsed_time(ev1), dev)
     clocks = sampler.stop() if (rank == 0 and sample_clocks) else None
     value = world * B * T * steps / (ms / 1e3)
@@ -331,7 +347,7 @@ def measure_training(wl, model, rank, local_rank, world, dev, steps, warmup, e2e
 
 def run_training(args, wl, model, cfg, rank, local_rank, world, dev):
     import torch.distributed as dist
-    rec = measure_training(wl, model, rank, local_rank, world, dev, args.steps, args.warmup)
+    rec = measure_training(wl, model, rank, local_rank, world, dev, args.steps, args.warmup, dump=args.dump_outputs)
     if rank == 0:
         line = {"metric": rec["metric"], "value": rec["value"], "unit": "tokens/s", "n_gpus": world, "steps": args.steps,
                 "warmup": rec["warmup"], "ms_per_step": rec["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -358,7 +374,13 @@ def main():
     ap.add_argument("--pool", type=int, default=6, help="distinct context batches rotated through")
     ap.add_argument("--profile-run", action="store_true",
                     help="for runs under ncu: only the device-resident timed loop (no clock pre/post roll, no e2e, no roofline legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "sat":
+        ap.error("--dump-outputs applies to --impl sat")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -416,8 +438,8 @@ def main():
 
     def loop(i):
         if beam > 1:
-            return model.beam_device(ctx_dev[i % pool], beam, T, 2)[0]
-        return model.loop_device(ctx_dev[i % pool], T)[0]
+            return model.beam_device(ctx_dev[i % pool], beam, T, 2)
+        return model.loop_device(ctx_dev[i % pool], T)[:1]
 
     for i in range(max(args.warmup, 3) + 2 * pool):       # warm-up also builds one CUDA graph per pool entry
         loop(i)
@@ -444,9 +466,12 @@ def main():
     with torch.cuda.stream(st):
         ev0.record(st)
         for i in range(args.steps):
-            loop(i)
+            last = loop(i)
         ev1.record(st)
     barrier()
+    if args.dump_outputs and rank == 0:      # (persistent buffers: dumped before any later loop overwrites them)
+        names = ("sentences", "lengths", "scores", "num_results", "complete") if beam > 1 else ("tokens",)
+        dump_outputs(args.dump_outputs, dict(zip(names, last)))
     ms = ev0.elapsed_time(ev1)
     launches = model.info("launches")
     if not args.profile_run:
